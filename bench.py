@@ -143,7 +143,7 @@ def cpu_baseline(inst, L, dtype=np.float32):
 def reference_threadmode(seconds=10):
     """The UNMODIFIED reference's own thread-mode solve (`pydcop -t T solve -a maxsum -d adhoc`, one Python thread
     per agent: GIL-bound, effectively one core) timed on THIS box's host: BASELINE.md 3.1 (C1, the reference's
-    graph_coloring_10_4_15_0.1.yml) and 3.2 (a C2-family instance with V = 100).  Reference = baseline/_ref, the
+    graph_coloring_10_4_15_0.1.yml) and 3.2 (a C2-family instance with V = 100).  Reference = oracle/_ref, the
     pip-installed copy of the source tree (oracle/ref_shim.py adds three import shims, edits nothing).  Returns a
     list of cpu_baseline entries (kind `reference-threadmode`); [] with a reason when the install is absent."""
     import subprocess
@@ -188,6 +188,27 @@ def reference_threadmode(seconds=10):
             except Exception as ex:  # noqa: BLE001 — a baseline must not cost the measured line
                 out.append({"kind": "reference-threadmode", "unavailable": f"{name}: {ex!r}"[:300]})
     return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write `arrays` (name -> numpy array) as out_dir/<name>.npy, floats in float32 / float64 and the rest as
+    float64.  When they add up to more than DUMP_LIMIT_BYTES, every array above an equal share of the limit is
+    replaced by the same seeded sample of its elements (sorted flat indices from default_rng(0)), so two runs
+    with the same arguments write comparable files."""
+    arrays = {k: np.ravel(v if v.dtype in (np.float32, np.float64) else v.astype(np.float64))
+              for k, v in arrays.items()}
+    if sum(a.nbytes for a in arrays.values()) > DUMP_LIMIT_BYTES:
+        share = DUMP_LIMIT_BYTES // len(arrays)
+        for k, a in arrays.items():
+            if a.nbytes > share:
+                keep = share // a.itemsize
+                arrays[k] = a[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def _partition_cache_path(inst, world, part):
@@ -361,7 +382,12 @@ def main():
                          "| c4 DSA 1M vars d=20 (variable updates/s) | mgm: MGM on the c4 instance")
     ap.add_argument("--profile", action="store_true",
                     help="lean run for ncu: init + warmup + steps back to back, no flush/e2e/JSON")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the assignment, its reported costs and the q / r messages "
+                         "the last timed step left as DIR/<name>.npy (c2 workload; N > 1: the assignment)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "c2" or args.impl != "b200" or args.profile):
+        ap.error("--dump-outputs writes the outputs of the timed c2 path (--impl b200, no --profile)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -482,6 +508,16 @@ def main():
         dist.barrier()
     launches = runner.launch_count - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:   # the state the last timed step left, read back outside the timed region
+        if world > 1:
+            out = {"value": runner.values()}    # collective: every rank takes part
+        else:
+            ft = np.float32 if args.precision == "f32" else np.float64
+            value, value_cost = runner.values()
+            q, r = runner.messages()
+            out = {"value": value, "value_cost": value_cost.astype(ft), "q": q.astype(ft), "r": r.astype(ft)}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, out)
     ms = sum(a.elapsed_time(b) for a, b in evs)
     if world > 1:
         t = torch.tensor([ms], device=dev, dtype=torch.float64)

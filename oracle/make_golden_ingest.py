@@ -59,6 +59,24 @@ def main():
     with open(path, "w") as f:
         json.dump(expected, f, indent=1, sort_keys=True)
     print("wrote", path, {k: (len(v["variables"]), len(v["constraints"])) for k, v in expected.items()})
+    # the reference's own test instances (its tests/instances/, copied to tests/golden/instances/): per file
+    # "<file>/meta" (JSON: external variables or not, declaration order of variables and constraints, sorted
+    # scopes) and "<file>/<constraint>" (the table, axes in sorted variable-name order)
+    import numpy as np
+    idir = os.path.join(ROOT, "tests", "golden", "instances")
+    out = {}
+    for fn in sorted(f for f in os.listdir(idir) if f.endswith((".yaml", ".yml"))):
+        dcop = load_dcop_from_file([os.path.join(idir, fn)])
+        meta = {"external_variables": bool(dcop.external_variables)}
+        if not dcop.external_variables:
+            d = describe(dcop)
+            meta.update(var_order=list(dcop.variables), con_order=list(dcop.constraints),
+                        scopes={n: c["scope"] for n, c in d["constraints"].items()})
+            out.update({f"{fn}/{n}": np.array(c["table"]) for n, c in d["constraints"].items()})
+        out[f"{fn}/meta"] = np.array(json.dumps(meta))
+    path = os.path.join(ROOT, "tests", "golden", "instances_expected.npz")
+    np.savez_compressed(path, **out)
+    print("wrote", path)
 
 
 if __name__ == "__main__":

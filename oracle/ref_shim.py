@@ -1,12 +1,11 @@
-"""Import shims that let the UNMODIFIED reference (pyDcop @ /root/reference) import under
-Python 3.12 / numpy 2 in the build container.  TEST INFRASTRUCTURE ONLY.
+"""Import shims that let the UNMODIFIED reference (pyDcop) import under Python 3.12 / numpy 2.
+TEST INFRASTRUCTURE ONLY.
 
-Only `oracle/make_golden.py` (fixture generation, build container only), the plugin tests and
-bench.py's `reference-threadmode` baseline use this; nothing in the product path imports it.
-/root/reference does not exist on the GPU box: there the reference is the unmodified copy that
-`python -m pip install --target baseline/_ref` made in the build container (git-ignored, shipped
-with the snapshot) — used by the drop-in test that runs the REAL engine under the reference's own
-orchestrator and by the timed thread-mode baseline, never by the product path.
+Only the golden generators under oracle/, the tests that run the reference and bench.py's
+`reference-threadmode` baseline use this; nothing in the product path imports it.  The reference is
+the copy oracle/install_reference.py installed into oracle/_ref/ (git-ignored, built by
+__graft_entry__.build()), else its source tree (PYDCOP_REFERENCE); the tests that need it skip
+where neither exists.
 
 Shims (SURVEY.md §8c):
   1. collections.Iterable/Mapping/... aliases (reference: pydcop/dcop/yamldcop.py:32, dcop.py:238)
@@ -19,12 +18,11 @@ import os
 import sys
 import types
 
-_REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-#: the unmodified reference: the source tree in the build container, else the copy `pip install --target
-#: baseline/_ref` made of it (git-ignored; it travels to the GPU box with the snapshot, __graft_entry__.build)
-INSTALLED_ROOT = os.path.join(_REPO, "baseline", "_ref")
-REFERENCE_ROOT = os.environ.get("PYDCOP_REFERENCE") or (
-    "/root/reference" if os.path.isdir("/root/reference/pydcop") else INSTALLED_ROOT)
+import install_reference
+
+#: the unmodified reference: the installed copy in oracle/_ref/, else the source tree it is installed from
+INSTALLED_ROOT = install_reference.TARGET
+REFERENCE_ROOT = INSTALLED_ROOT if install_reference.installed() else install_reference.SOURCE
 
 
 def reference_available() -> bool:

@@ -1,8 +1,7 @@
 """GPU: ONE true drop-in run — the UNMODIFIED reference CLI (`pydcop solve`: argument parsing, distribution,
 orchestrator, agents in thread mode, JSON result) with `--algo maxsum_gpu` / `dsa_gpu` / `mgm_gpu` and the REAL
-engine behind the proxies (no oracle in the seam).  On the GPU box the reference is the unmodified copy that
-`pip install --target baseline/_ref` made in the build container (__graft_entry__.install_reference; it ships with
-the snapshot); the three import shims of oracle/ref_shim.py are installed before `pydcop` is imported, nothing in
+engine behind the proxies (no oracle in the seam).  The reference is the unmodified copy that
+oracle/install_reference.py installed into oracle/_ref/ (__graft_entry__.build()); the three import shims of oracle/ref_shim.py are installed before `pydcop` is imported, nothing in
 the reference is edited.  Checked: status FINISHED (every graph node finished, orchestrator.py:898-913), the cycle
 count, and the assignment against the CPU oracle on the same problem (algorithms/__init__.py:527-566 loads the
 module by name)."""
@@ -19,7 +18,7 @@ import ref_shim
 
 pytestmark = [pytest.mark.gpu,
               pytest.mark.skipif(not ref_shim.reference_available(),
-                                 reason="no reference: neither /root/reference nor baseline/_ref")]
+                                 reason="no reference: oracle/_ref/ not installed")]
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 INSTANCES = os.path.join(ref_shim.REFERENCE_ROOT, "tests", "instances")

@@ -1,5 +1,5 @@
-"""The pyDcop drop-in boundary, exercised with the UNMODIFIED reference in thread mode (build
-container only: needs /root/reference).  There is no GPU here, so the end-to-end runs put the CPU
+"""The pyDcop drop-in boundary, exercised with the UNMODIFIED reference in thread mode (the copy in
+oracle/_ref/, see oracle/install_reference.py).  There is no GPU here, so the end-to-end runs put the CPU
 oracle behind the session's engine seam — that checks the plugin plumbing (registration, closure
 detection, value reporting, cycle counting, FINISHED status), not the kernels; without the seam
 the product path must fail loudly instead of falling back."""
@@ -13,7 +13,7 @@ import oracle as orc
 import ref_shim
 
 pytestmark = pytest.mark.skipif(not ref_shim.reference_available(),
-                                reason="reference tree not present (GPU box)")
+                                reason="no reference: oracle/_ref/ not installed")
 
 INSTANCES = os.path.join(ref_shim.REFERENCE_ROOT, "tests", "instances")
 
